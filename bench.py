@@ -1,8 +1,12 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the CodeFormer hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes what the last timed step returned to its caller as DIR/<name>.npy (float32): out, logits and
+lq_feat of CodeFormer.forward on one GPU, the gathered out on N GPUs.  Inputs and weights are seeded, so two builds of the
+project run with the same arguments can be compared output for output.
 
 A "step" = one CodeFormer.forward(x, w=0.5, adain=True) over one batch of 32 synthetic 512x512 faces per
 GPU (BASELINE.json configs[1]; N GPUs = configs[4], 32 faces/GPU, weak scaling) followed -- for N>1 -- by
@@ -239,6 +243,37 @@ def dominant_kernel_roofline(torch, cb, batch, peaks, peak_kind):
                     'ms_per_launch': ms64, 'frac': flops / (ms64 * 1e-3) / 1e12 / peaks['bf16_tflops']}}}
 
 
+DUMP_BUDGET = 64 * 10**6        # bytes of all .npy files of one --dump-outputs
+DUMP_RESERVE = 16 * 10**6       # kept for each array not yet written
+NPY_HEADER = 128                # np.save header of a 1-D or 3-D float32 array
+
+
+def dump_outputs(torch, arrays, out_dir, seed=0):
+    """Write each tensor of `arrays` (name -> tensor) as out_dir/<name>.npy in float32, within DUMP_BUDGET bytes in all.
+    Smallest first, an array is written whole, in its own shape, while that leaves DUMP_RESERVE bytes for each array still
+    to come; an array that does not fit is written as a fixed sample of its flattened elements: the sorted positions
+    np.random.default_rng(seed).choice(numel, n, replace=False), n filling its share of the budget that is left.
+    -> {name: {'shape', 'elements', 'sample_seed'}} (sample_seed None: the whole array)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    items = sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    left, info = DUMP_BUDGET, {}
+    for k, (name, t) in enumerate(items):
+        rest = len(items) - 1 - k
+        flat = t.detach().reshape(-1)
+        if NPY_HEADER + 4 * flat.numel() <= left - rest * DUMP_RESERVE:
+            a, sample_seed = t.detach().float().cpu().numpy(), None
+        else:
+            n = (left // (rest + 1) - NPY_HEADER) // 4
+            at = np.sort(np.random.default_rng(seed).choice(flat.numel(), n, replace=False))
+            a, sample_seed = flat[torch.from_numpy(at).to(flat.device)].float().cpu().numpy(), seed
+        path = os.path.join(out_dir, name + '.npy')
+        np.save(path, a)
+        left -= os.path.getsize(path)
+        info[name] = {'shape': list(t.shape), 'elements': int(a.size), 'sample_seed': sample_seed}
+    return info
+
+
 def _median_ms(torch, fn, iters, warm=3):
     for _ in range(warm):
         fn()
@@ -349,15 +384,18 @@ def run_b200(args):
     sg = StreamedGather() if world > 1 else None
 
     def step(i):
-        out = net(xs[i % 2], w=0.5, adain=True)[0]
+        """-> the arrays the caller of the path receives (name -> tensor); on N GPUs the gathered `out`, which the
+        asynchronous gather delivers only at the next submit / flush."""
+        out, logits, lq_feat = net(xs[i % 2], w=0.5, adain=True)
         if world > 1:
             # the one collective of the path (section 8e), off the critical path: issued asynchronously after the forward, it
             # completes on NCCL's stream while the next step's forward runs (parallel.StreamedGather); the timed region ends
             # with flush(), so every gather is inside it.  --gather-chunks 2 selects the half-batch pipeline instead.
             if args.gather_chunks > 1:
-                return pipelined_forward_gather(net, xs[i % 2], gathered, chunks=args.gather_chunks, w=0.5, adain=True)[1]
+                return {'out': pipelined_forward_gather(net, xs[i % 2], gathered, chunks=args.gather_chunks, w=0.5, adain=True)[0]}
             sg.submit(out)
-        return out
+            return {}
+        return {'out': out, 'logits': logits, 'lq_feat': lq_feat}
 
     def barrier():
         if world > 1:
@@ -376,9 +414,12 @@ def run_b200(args):
     barrier()
     e0.record()
     for i in range(args.steps):
-        step(i)
+        last = None                                          # a step's outputs are released before the next step runs
+        last = step(i)
     if sg is not None:
-        sg.flush()                                           # the last gather completes inside the timed region
+        done = sg.flush()                                    # the last gather completes inside the timed region
+        if done is not None:
+            last = {'out': done}
     e1.record()
     barrier()
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
@@ -388,6 +429,8 @@ def run_b200(args):
     clocks = sampler.stop() if sampler else None
     ms_total = float(ms.item())
     value = world * batch * args.steps / (ms_total * 1e-3)
+    dumped = dump_outputs(torch, last, args.dump_outputs) if args.dump_outputs and rank == 0 else None
+    del last
 
     # ---- multi-GPU evidence (section 8d config 5): the gathered tensor holds every rank's shard bit for bit, and where the
     # step time goes on each rank (forward alone, gather alone; CUDA events)
@@ -488,6 +531,8 @@ def run_b200(args):
                 'gpu_launches': int(launches), 'clocks': clocks, 'roofline': roof}
         if e2e_u8:
             line['e2e_u8'] = e2e_u8
+        if dumped:
+            line['dump_outputs'] = {'dir': args.dump_outputs, 'arrays': dumped}
         if multi:
             line['multi_gpu'] = multi
             line['gather_bit_identical'] = multi['gather_bit_identical']
@@ -516,7 +561,13 @@ def main():
     ap.add_argument('--no-extras', action='store_true', help='skip BASELINE configs 1/3/4 (latency, VQ microbench, VQAE B=64)')
     ap.add_argument('--gather-chunks', type=int, default=1,
                     help='N>1: 1 = asynchronous gather overlapping the next step (default); >1 = half-batch pipeline inside a step')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB in all)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the b200 path only')
     if args.impl == 'reference':
         run_reference(args)
     else:

@@ -21,6 +21,11 @@ Files
                             tensor2img(min_max=(-1,1)).astype(uint8) of the reference on a u8 face that holds every byte
                             value in every channel and on an fp32 tensor that holds every rounding half-way point
                             (`python oracle/gen_golden.py plumbing` regenerates only this file)
+  reference_checks.npz      small direct checks of the reference's own modules: state-dict keys and shapes of CodeFormer,
+                            RRDBNet and ParseNet; VectorQuantizer on 4 config-3 latents; one TransformerSALayer (every 16th
+                            token of its output); img2tensor/tensor2img on a 32x48 face; RealESRGANer.enhance around
+                            ToyUpsampler for every ESR_CASES entry
+                            (`python oracle/gen_golden.py reference_checks` regenerates only this file)
 """
 import os
 import sys
@@ -151,7 +156,103 @@ def gen_parsenet():
                         classes=mask.argmax(1).numpy().astype(np.uint8), margin=(top2[:, 0] - top2[:, 1]).numpy().astype(np.float16))
 
 
+class ToyUpsampler(torch.nn.Module):
+    """A cheap x2 'upsampler' with a 5x5 receptive field: enough to make tiling / padding mistakes visible."""
+
+    def __init__(self):
+        super().__init__()
+        g = torch.Generator().manual_seed(3)
+        self.w = torch.nn.Parameter(torch.randn(3, 3, 5, 5, generator=g) * 0.1)
+
+    def forward(self, x):
+        y = torch.nn.functional.conv2d(x, self.w, padding=2)
+        return torch.nn.functional.interpolate(y, scale_factor=2, mode='nearest')
+
+
+ESR_CASES = [(0, 0, (37, 45, 3)), (16, 0, (37, 45, 3)), (16, 10, (50, 33, 3)), (20, 4, (41, 41)), (16, 0, (30, 34, 4))]   # tile, pre_pad, image shape
+
+
+def esr_image(shape):
+    return np.random.default_rng(7).integers(0, 256, shape, dtype=np.uint8)
+
+
+def esr_key(tile, pre_pad, shape):
+    return f'esr_t{tile}_p{pre_pad}_' + 'x'.join(map(str, shape))
+
+
+def transformer_layer_inputs():
+    """Seeded parameters of one TransformerSALayer(512, 8, 1024) (the ft_layers.0 entries of the CodeFormer spec, prefix 'L'),
+    a [256, 2, 512] token sequence and its position embedding."""
+    spec = S.codeformer_spec()
+    sub = type(spec)((k, v) for k, v in spec.items() if k.startswith('ft_layers.0.'))
+    sd = {'L.' + k[len('ft_layers.0.'):]: v for k, v in S.random_state_dict(sub, 3).items()}
+    g = torch.Generator().manual_seed(3)
+    t = torch.randn(256, 2, 512, generator=g)
+    pos = torch.randn(256, 2, 512, generator=g) * 0.02
+    return sd, t, pos
+
+
+def plumbing_small_inputs():
+    """A random 32x48 BGR face and a [1,3,32,48] network output (values beyond +-1 included)."""
+    rng = np.random.default_rng(11)
+    face = rng.integers(0, 256, (32, 48, 3), dtype=np.uint8)
+    out = (rng.standard_normal((1, 3, 32, 48)) * 0.8).astype(np.float32)
+    return face, out
+
+
+def state_dict_table(sd):
+    """-> (keys, shapes as 'd0,d1,...', dtypes) string arrays of a state dict."""
+    return (np.array(list(sd.keys())), np.array([','.join(map(str, v.shape)) for v in sd.values()]),
+            np.array([str(v.dtype) for v in sd.values()]))
+
+
+def gen_reference_checks():
+    """tests/golden/reference_checks.npz: what the tests used to compare against the reference modules imported live."""
+    CodeFormer, _, VQ, _ = ref_shim.load()
+    torch.set_grad_enabled(False)
+    res = {}
+    for name, net in (('codeformer', CodeFormer()),
+                      ('rrdbnet', load_ref_rrdbnet()(3, 3, scale=2, num_feat=64, num_block=23, num_grow_ch=32)),
+                      ('parsenet', load_ref_parsenet()(in_size=512, out_size=512, parsing_ch=19))):
+        res[name + '_keys'], res[name + '_shapes'], res[name + '_dtypes'] = state_dict_table(net.state_dict())
+
+    E, z = vq_micro_inputs('B')
+    m = VQ(1024, 256, 0.25)
+    m.embedding.weight.data.copy_(E)
+    zq, _, st = m(z[:4])
+    sample = np.sort(np.random.default_rng(0).choice(zq.numel(), 4096, replace=False))
+    res.update(vq4_idx=st['min_encoding_indices'].numpy(), vq4_zq_sample=zq.reshape(-1)[torch.from_numpy(sample)].numpy(),
+               vq4_sample_at=sample)
+
+    from basicsr.archs.codeformer_arch import TransformerSALayer
+    sd, t, pos = transformer_layer_inputs()
+    layer = TransformerSALayer(512, 8, 1024).eval()
+    layer.load_state_dict({k[2:]: v for k, v in sd.items()}, strict=True)
+    res['sa_layer_out_s16'] = layer(t, query_pos=pos)[::16].numpy()
+
+    from basicsr.utils import img2tensor, tensor2img
+    from torchvision.transforms.functional import normalize
+    face, out = plumbing_small_inputs()
+    x = img2tensor(face / 255., bgr2rgb=True, float32=True)
+    normalize(x, (0.5, 0.5, 0.5), (0.5, 0.5, 0.5), inplace=True)
+    res.update(plumbing_small_x=x.numpy(),
+               plumbing_small_restored=tensor2img(torch.from_numpy(out.copy()), rgb2bgr=True, min_max=(-1, 1)).astype('uint8'))
+
+    from basicsr.utils.realesrgan_utils import RealESRGANer
+    model = ToyUpsampler().eval()
+    for tile, pre_pad, shape in ESR_CASES:
+        er = RealESRGANer.__new__(RealESRGANer)              # the reference constructor insists on loading a checkpoint file
+        er.scale, er.tile_size, er.tile_pad, er.pre_pad, er.mod_scale, er.half = 2, tile, 6, pre_pad, None, False
+        er.device, er.model = torch.device('cpu'), model
+        o, mode = er.enhance(esr_image(shape), outscale=2)
+        res[esr_key(tile, pre_pad, shape)], res[esr_key(tile, pre_pad, shape) + '_mode'] = o, np.array(mode)
+    np.savez_compressed(os.path.join(OUT, 'reference_checks.npz'), **res)
+
+
 def main():
+    if len(sys.argv) > 1 and sys.argv[1] == 'reference_checks':
+        gen_reference_checks()
+        return
     if len(sys.argv) > 1 and sys.argv[1] == 'parsenet':
         gen_parsenet()
         return
@@ -215,6 +316,7 @@ def main():
     gen_plumbing()
     gen_rrdbnet()
     gen_parsenet()
+    gen_reference_checks()
     for f in sorted(os.listdir(OUT)):
         print(f, os.path.getsize(os.path.join(OUT, f)) // 1024, 'KiB')
 

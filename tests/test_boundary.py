@@ -8,8 +8,7 @@ import torch
 
 import codeformer_b200 as cb
 from codeformer_b200 import _lib, spec as S
-from oracle import ref_shim
-from tests.util import ROOT
+from tests.util import ROOT, golden
 
 
 def test_state_dict_contract_codeformer():
@@ -43,13 +42,12 @@ def test_state_dict_contract_vqae():
         cb.VQAutoEncoder(512, 64, [1, 2, 2, 4, 4, 8], 'gumbel')
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason='/root/reference not present (GPU box)')
 def test_keys_equal_live_reference():
-    CodeFormer, VQAE, _, _ = ref_shim.load()
-    ref = CodeFormer().state_dict()
+    """Keys, order and shapes of the reference's CodeFormer() state dict (tests/golden/reference_checks.npz)."""
+    g = golden('reference_checks.npz')
     ours = cb.CodeFormer().state_dict()
-    assert list(ref.keys()) == list(ours.keys())
-    assert all(ref[k].shape == ours[k].shape for k in ref)
+    assert list(g['codeformer_keys']) == list(ours.keys())
+    assert list(g['codeformer_shapes']) == [','.join(map(str, v.shape)) for v in ours.values()]
 
 
 def test_registry_interface():
@@ -94,6 +92,9 @@ def test_host_planning_without_gpu():
     net = cb.CodeFormer()
     h = ctypes.c_void_p(lib.cfb_net_create(ctypes.byref(net._cfb_config())))
     assert h
+    # the fp32 engine: the plan cfb_net_create picks when no tcgen05 device is present, here on every machine (on a B200
+    # the default engine plans the tensor-core path, whose arena is laid out differently)
+    assert lib.cfb_net_set_engine(h, 1) == 0
     w1, w8 = lib.cfb_workspace_bytes(h, 1), lib.cfb_workspace_bytes(h, 8)
     assert 0 < w1 < w8 < 8 * w1 + (1 << 20)
     assert lib.cfb_workspace_bytes(h, 0) >= 0
@@ -123,17 +124,33 @@ def test_product_never_imports_oracle():
                 assert 'oracle' not in src.replace('no CPU fallback', ''), f'{f} mentions the oracle'
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason='/root/reference not present (GPU box)')
+class _BasicsrRegistry:
+    """The behaviour of basicsr's Registry (basicsr/utils/registry.py) that install() relies on: the classes live in a private
+    name -> class dict ``_obj_map``, ``register`` asserts when the name is already taken, ``get`` raises KeyError when absent."""
+
+    def __init__(self):
+        self._obj_map = {}
+
+    def register(self, obj):
+        assert obj.__name__ not in self._obj_map, f'{obj.__name__} is already registered'
+        self._obj_map[obj.__name__] = obj
+
+    def get(self, name):
+        if self._obj_map.get(name) is None:
+            raise KeyError(name)
+        return self._obj_map[name]
+
+
 def test_install_replaces_entries_of_the_reference_registry():
-    """`install()` must swap the two entries of the reference's own ARCH_REGISTRY in place (registry.py:39 would assert
+    """`install()` must swap the two entries of the reference's ARCH_REGISTRY in place (registry.py:39 would assert
     on a second registration), after which the reference's lookup returns the B200 classes."""
-    _, _, _, REG = ref_shim.load()
-    before = REG.get('CodeFormer')
-    try:
-        cb.install(REG)
-        assert REG.get('CodeFormer') is cb.CodeFormer and REG.get('VQAutoEncoder') is cb.VQAutoEncoder
-        net = REG.get('CodeFormer')(dim_embd=512, codebook_size=1024, n_head=8, n_layers=9,
-                                    connect_list=['32', '64', '128', '256'])
-        assert len(net.state_dict()) == 515
-    finally:
-        REG._obj_map['CodeFormer'] = before
+    REG = _BasicsrRegistry()
+    for name in ('CodeFormer', 'VQAutoEncoder'):
+        REG.register(type(name, (torch.nn.Module,), {}))         # the reference's own classes, registered at import
+    with pytest.raises(AssertionError):
+        REG.register(cb.CodeFormer)
+    assert cb.install(REG) is REG
+    assert REG.get('CodeFormer') is cb.CodeFormer and REG.get('VQAutoEncoder') is cb.VQAutoEncoder
+    net = REG.get('CodeFormer')(dim_embd=512, codebook_size=1024, n_head=8, n_layers=9,
+                                connect_list=['32', '64', '128', '256'])
+    assert len(net.state_dict()) == 515

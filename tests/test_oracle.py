@@ -1,12 +1,12 @@
 """The oracle (oracle/codeformer_oracle.py) against the golden vectors produced by the UNMODIFIED
-reference (oracle/gen_golden.py) and, when /root/reference is present, against the live reference."""
+reference (oracle/gen_golden.py)."""
 import numpy as np
 import pytest
 import torch
 
 from tests.util import faces_input, golden, maxabs, vq_micro_inputs
 from oracle import codeformer_oracle as O
-from oracle import ref_shim
+from oracle import gen_golden as GG
 from codeformer_b200 import spec as S
 
 torch.set_grad_enabled(False)
@@ -65,23 +65,16 @@ def test_vq_micro_matches_reference_golden(case):
     assert abs(float(loss) - float(g[f'{case}_loss'])) < 1e-5 * max(1.0, float(g[f'{case}_loss']))
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason='/root/reference not present (GPU box)')
 def test_oracle_equals_live_reference_small():
-    """Live check of the restatement, on a case that is cheap: VectorQuantizer + one TransformerSALayer."""
-    CodeFormer, VQAE, VQ, _ = ref_shim.load()
+    """The restatement against the reference modules on a cheap case: VectorQuantizer on 4 latents + one TransformerSALayer
+    (tests/golden/reference_checks.npz)."""
+    g = golden('reference_checks.npz')
     E, z = vq_micro_inputs('B')
-    m = VQ(1024, 256, 0.25)
-    m.embedding.weight.data.copy_(E)
-    a = m(z[:4])
-    b = O.vq_forward({'quantize.embedding.weight': E}, z[:4])
-    assert torch.equal(a[2]['min_encoding_indices'], b[2]['min_encoding_indices']) and torch.equal(a[0], b[0])
-    from basicsr.archs.codeformer_arch import TransformerSALayer
-    torch.manual_seed(3)
-    layer = TransformerSALayer(512, 8, 1024).eval()
-    sd = {'L.' + k: v for k, v in layer.state_dict().items()}
-    t = torch.randn(256, 2, 512)
-    pos = torch.randn(256, 2, 512) * 0.02
-    assert maxabs(layer(t, query_pos=pos), O.transformer_layer(sd, 'L', t, pos, 8)) < 5e-6
+    zq, _, st = O.vq_forward({'quantize.embedding.weight': E}, z[:4])
+    assert np.array_equal(st['min_encoding_indices'].numpy(), g['vq4_idx'])
+    assert np.array_equal(zq.reshape(-1)[torch.from_numpy(g['vq4_sample_at'])].numpy(), g['vq4_zq_sample'])
+    sd, t, pos = GG.transformer_layer_inputs()
+    assert maxabs(O.transformer_layer(sd, 'L', t, pos, 8)[::16], g['sa_layer_out_s16']) < 5e-6
 
 
 def test_plumbing_matches_reference_golden():
@@ -95,17 +88,10 @@ def test_plumbing_matches_reference_golden():
     assert np.array_equal(P.output_to_face(P.face_to_input(g['face_bgr'][None])), g['face_bgr'][None])
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason='/root/reference not present (GPU box)')
 def test_plumbing_equals_live_reference():
+    """img2tensor+normalize and tensor2img of the reference on a random 32x48 face (tests/golden/reference_checks.npz)."""
     from oracle import plumbing_oracle as P
-    ref_shim.load()
-    from basicsr.utils import img2tensor, tensor2img
-    from torchvision.transforms.functional import normalize
-    rng = np.random.default_rng(11)
-    face = rng.integers(0, 256, (32, 48, 3), dtype=np.uint8)
-    t = img2tensor(face / 255., bgr2rgb=True, float32=True)
-    normalize(t, (0.5, 0.5, 0.5), (0.5, 0.5, 0.5), inplace=True)
-    assert np.array_equal(t.numpy(), P.face_to_input(face[None])[0])
-    out = torch.from_numpy((rng.standard_normal((1, 3, 32, 48)) * 0.8).astype(np.float32))
-    r = tensor2img(out.clone(), rgb2bgr=True, min_max=(-1, 1)).astype('uint8')
-    assert np.array_equal(r, P.output_to_face(out.numpy())[0])
+    g = golden('reference_checks.npz')
+    face, out = GG.plumbing_small_inputs()
+    assert np.array_equal(g['plumbing_small_x'], P.face_to_input(face[None])[0])
+    assert np.array_equal(g['plumbing_small_restored'], P.output_to_face(out)[0])

@@ -1,6 +1,6 @@
 """not gpu: the oracles of the caller-side networks (SURVEY.md section 8 rows f3 / f4) against the golden vectors written by the
-UNMODIFIED reference (oracle/gen_golden.py) and -- when /root/reference is present -- against the live reference classes;
-plus the host logic of the RealESRGANer front-end (tile plan, padding, colour handling) against the reference's."""
+UNMODIFIED reference (oracle/gen_golden.py); plus the host logic of the RealESRGANer front-end (tile plan, padding, colour
+handling) against the reference's."""
 import numpy as np
 import pytest
 import torch
@@ -8,7 +8,6 @@ import torch
 import codeformer_b200 as cb
 from codeformer_b200 import spec as S
 from oracle import gen_golden as GG
-from oracle import ref_shim
 from oracle import rrdbnet_oracle as RO
 from tests.util import golden, maxabs
 
@@ -31,42 +30,24 @@ def test_rrdbnet_state_dict_contract():
     ours.load_state_dict(S.random_state_dict(S.rrdbnet_spec(3, 3, 2, 64, 23, 32), 5), strict=True)
     with pytest.raises(RuntimeError, match='no CPU fallback'):
         ours(torch.zeros(1, 3, 8, 8))
-    if ref_shim.available():
-        ref = GG.load_ref_rrdbnet()(3, 3, scale=2, num_feat=64, num_block=23, num_grow_ch=32).state_dict()
-        mine = ours.state_dict()
-        assert list(ref.keys()) == list(mine.keys()) and all(ref[k].shape == mine[k].shape for k in ref)
+    g = golden('reference_checks.npz')
+    mine = ours.state_dict()
+    assert list(g['rrdbnet_keys']) == list(mine.keys())
+    assert list(g['rrdbnet_shapes']) == [','.join(map(str, v.shape)) for v in mine.values()]
 
 
-class _Toy(torch.nn.Module):
-    """A cheap x2 'upsampler' with a 5x5 receptive field: enough to make tiling / padding mistakes visible."""
-
-    def __init__(self):
-        super().__init__()
-        g = torch.Generator().manual_seed(3)
-        self.w = torch.nn.Parameter(torch.randn(3, 3, 5, 5, generator=g) * 0.1)
-
-    def forward(self, x):
-        y = torch.nn.functional.conv2d(x, self.w, padding=2)
-        return torch.nn.functional.interpolate(y, scale_factor=2, mode='nearest')
+_Toy = GG.ToyUpsampler
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason='/root/reference not present (GPU box)')
-@pytest.mark.parametrize('tile,pre_pad,shape', [(0, 0, (37, 45, 3)), (16, 0, (37, 45, 3)), (16, 10, (50, 33, 3)), (20, 4, (41, 41)),
-                                               (16, 0, (30, 34, 4))])
+@pytest.mark.parametrize('tile,pre_pad,shape', GG.ESR_CASES)
 def test_realesrganer_front_end_equals_the_reference(tile, pre_pad, shape):
     """enhance(): colour handling, reflect pre/mod padding, the tile loop and the crop-back, bit for bit against the
-    reference's RealESRGANer around the same (CPU) model (realesrgan_utils.py:71-250)."""
-    ref_shim.load()
-    from basicsr.utils.realesrgan_utils import RealESRGANer as RefER
-    rng = np.random.default_rng(7)
-    img = rng.integers(0, 256, shape, dtype=np.uint8)
+    reference's RealESRGANer around the same (CPU) model (realesrgan_utils.py:71-250; tests/golden/reference_checks.npz)."""
     model = _Toy().eval()
     ours = cb.RealESRGANer(scale=2, model_path=None, model=model, tile=tile, tile_pad=6, pre_pad=pre_pad, device='cpu')
-    ref = RefER.__new__(RefER)                     # the reference constructor insists on loading a checkpoint file
-    ref.scale, ref.tile_size, ref.tile_pad, ref.pre_pad, ref.mod_scale, ref.half = 2, tile, 6, pre_pad, None, False
-    ref.device, ref.model = torch.device('cpu'), model
-    o1, m1 = ours.enhance(img, outscale=2)
-    o2, m2 = ref.enhance(img, outscale=2)
+    o1, m1 = ours.enhance(GG.esr_image(shape), outscale=2)
+    g = golden('reference_checks.npz')
+    o2, m2 = g[GG.esr_key(tile, pre_pad, shape)], str(g[GG.esr_key(tile, pre_pad, shape) + '_mode'])
     assert m1 == m2 and o1.dtype == o2.dtype and o1.shape == o2.shape
     assert np.array_equal(o1, o2)
 
@@ -108,6 +89,7 @@ def test_parsenet_state_dict_contract():
         net.eval()(torch.zeros(1, 3, 64, 64))
     with pytest.raises(RuntimeError, match='inference-only'):
         net.train()
-    if ref_shim.available():
-        ref = GG.load_ref_parsenet()(in_size=512, out_size=512, parsing_ch=19).state_dict()
-        assert list(ref.keys()) == list(sd.keys()) and all(ref[k].shape == sd[k].shape and ref[k].dtype == sd[k].dtype for k in ref)
+    g = golden('reference_checks.npz')
+    assert list(g['parsenet_keys']) == list(sd.keys())
+    assert list(g['parsenet_shapes']) == [','.join(map(str, v.shape)) for v in sd.values()]
+    assert list(g['parsenet_dtypes']) == [str(v.dtype) for v in sd.values()]
